@@ -9,8 +9,9 @@ region and are reported in `config`.
   python bench.py --gpus N --steps K --warmup W        (N > 1: launched under torch.distributed.run, one rank per GPU)
   python bench.py --impl reference ...                 (CPU port of the reference path on the host cores)
   python bench.py --preset q0.6 | asr0.6               (BASELINE.json configs 2 and 4; default vl2 = config 3, the metric)
+  python bench.py ... --dump-outputs DIR               (also write the timed call's tokens and last-step logits as .npy)
 
-value  = K / (CUDA-event time of K launches on the library's stream, max over ranks)   -- inputs resident in HBM
+value  = K / (CUDA-event time of K launches on the library's stream, max over ranks)   -- inputs resident in HBM, one timed window of K steps
 e2e    = K / wall time of K aha_b200_forward_step calls (host token in, host argmax out every step)
 N > 1:  `value` is N independent replicas (one request per GPU, no data-path collective, "scaling": "weak"); the SAME
         invocation then runs ONE request tensor-parallel over the N GPUs (heads / MLP rows sharded, partial sums exchanged
@@ -229,6 +230,14 @@ def emit(line):
         os.write(_REAL_STDOUT, data)
 
 
+def dump_outputs(out_dir, r):
+    """The timed call's results: the greedy ids of its K steps (what decode_steps returns) and the logits of the last step
+    (what forward_step returns for it), float64 / float32, under 1 MB together for every preset."""
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "decode_tokens.npy"), np.asarray(r["timed_tokens"], np.float64))
+    np.save(os.path.join(out_dir, "last_step_logits.npy"), np.asarray(r["last_logits"], np.float32))
+
+
 def ncu_traffic(preset):
     """dram__bytes_read.sum + dram__bytes_write.sum of ONE fused decode-step launch from the committed `ncu --set full`
     summary of this workload (a citation of a capture under profiles/, not a measurement of this run)."""
@@ -301,7 +310,7 @@ def measure_batch(m, wl, synth, n_req=8, n_prompt=128, n_gen=64):
             "note": "new design (SURVEY 8f rank 4): the reference serves one request at a time; batched CUDA-core GEMV + per-sequence decode attention, one CUDA graph per batch composition"}
 
 
-def measure(m, wl, cfg, synth, K, W, reps, barrier, want_e2e=True):
+def measure(m, wl, cfg, synth, K, W, barrier, want_e2e=True, want_last_logits=False):
     """prefill once, then time K fused decode steps (device-resident) and K forward_step calls (e2e)."""
     ids, data = make_inputs(m, wl, cfg, synth)
     S = len(ids)
@@ -314,16 +323,19 @@ def measure(m, wl, cfg, synth, K, W, reps, barrier, want_e2e=True):
     warm = m.decode_steps(tok, S, W)
     m.reset_stats()
     barrier()
-    best_ms, out = None, None
     wall0 = time.perf_counter()
-    for _ in range(reps):
-        out, ms = m.decode_steps(warm[-1], S + W, K, timed=True)
-        best_ms = ms if best_ms is None else min(best_ms, ms)
+    out, ms = m.decode_steps(warm[-1], S + W, K, timed=True)
     barrier()
     wall_value = time.perf_counter() - wall0
     st = m.stats()
-    res = dict(S=S, usage=usage, rope_delta=rope_delta, best_ms=best_ms, tokens=[tok] + list(warm) + list(out), wall_value=wall_value,
-               launches=st["kernel_launches"] // reps, stats=st)
+    res = dict(S=S, usage=usage, rope_delta=rope_delta, ms=ms, tokens=[tok] + list(warm) + list(out), timed_tokens=out, wall_value=wall_value,
+               launches=st["kernel_launches"], stats=st)
+    if want_last_logits:
+        # the last timed step once more, on the cache it saw (before the e2e loop below overwrites those positions): the same kernel on the
+        # same inputs, so these are the logits that step computed, as forward_step hands them to a caller
+        prev = out[-2] if K > 1 else warm[-1]
+        res["last_logits"] = m.forward_step(np.array([prev], np.uint32), S + W + K - 1)
+        assert m.last_argmax == out[-1], "re-running the last timed step gave a different token"
     if want_e2e:
         t = out[-1]
         barrier()
@@ -371,7 +383,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-tp", action="store_true", help="N > 1: skip the tensor-parallel (strong scaling) arm")
     ap.add_argument("--decode-impl", type=int, default=int(os.environ.get("AHA_DECODE_IMPL", "0")))
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last of them computed to DIR/*.npy "
+                                                              "(rank 0; seeded inputs, so two builds can be compared output for output)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the B200 arm")
     K, W = args.steps, max(args.warmup, 3)
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -437,15 +455,16 @@ def main():
     t0 = time.time()
     m = B200Model(wl["kind"], cfg, wts, **kw)
     log(f"[rank {rank}] model created in {time.time() - t0:.1f}s")
-    reps = max(1, int(os.environ.get("AHA_BENCH_REPS", "3")))
     sampler = ClockSampler(local_rank)
     sampler.start()
     time.sleep(0.3)
-    r = measure(m, wl, cfg, synth, K, W, reps, barrier)
+    r = measure(m, wl, cfg, synth, K, W, barrier, want_last_logits=args.dump_outputs is not None)
     clocks = sampler.stop()
     assert r["S"] == S
+    if args.dump_outputs is not None and rank == 0:
+        dump_outputs(args.dump_outputs, r)
     usage, st = r["usage"], r["stats"]
-    log(f"[rank {rank}] prefill {usage['prompt_secs']:.3f}s (tower {usage['vision_secs']:.3f}s); decode {r['best_ms'] / K:.4f} ms/step")
+    log(f"[rank {rank}] prefill {usage['prompt_secs']:.3f}s (tower {usage['vision_secs']:.3f}s); decode {r['ms'] / K:.4f} ms/step")
 
     # ---- per-op twin kernels timed alone (where the step's bytes go), CUDA events
     peak, peak_src = measured_peaks()
@@ -455,7 +474,7 @@ def main():
         kernels[name] = {"avg_us": kms * 1e3, "bytes": kb, "gbps": kb / (kms * 1e-3) / 1e9}
     fused = st["kernels_per_decode_step"] == 1
     dev = f"cuda:{local_rank}"
-    value, max_ms = dist_util.aggregate_throughput(K, r["best_ms"], world, dist, dev)        # units of all ranks / slowest rank
+    value, max_ms = dist_util.aggregate_throughput(K, r["ms"], world, dist, dev)        # units of all ranks / slowest rank
     e2e_val, _ = dist_util.aggregate_throughput(K, r["e2e_s"] * 1e3, world, dist, dev)
     step_ms = max_ms / K
     avg_ctx = S + W + (K - 1) / 2.0 + 1
@@ -475,8 +494,8 @@ def main():
           uid = [nccl_unique_id() if rank == 0 else None]
           dist.broadcast_object_list(uid, src=0)
           mt = B200Model(wl["kind"], cfg, wts, tp_rank=rank, tp_world=world, tp_unique_id=uid[0], **kw)
-          rt = measure(mt, wl, cfg, synth, K, W, reps, barrier, want_e2e=True)
-          tp_ms = dist_util.reduce_max(rt["best_ms"], dist, dev)
+          rt = measure(mt, wl, cfg, synth, K, W, barrier, want_e2e=True)
+          tp_ms = dist_util.reduce_max(rt["ms"], dist, dev)
           tp_e2e = dist_util.reduce_max(rt["e2e_s"], dist, dev)
           n_cmp = min(len(single_tokens), len(rt["tokens"]))
           same = [int(a == b) for a, b in zip(single_tokens[:n_cmp], rt["tokens"][:n_cmp])]
@@ -493,7 +512,7 @@ def main():
                     "bytes_per_rank_per_step": tp_bytes, "gbps_per_rank": tp_bytes / (tp_ms / K * 1e-3) / 1e9,
                     "prefill_secs": rt["usage"]["prompt_secs"],
                     "tp_parity": ("ok" if first_diff is None else f"first differing greedy token at position {first_diff} of {n_cmp} (fp32 summation order differs between TP sizes)"),
-                    "ranks_agree": bool(ranks_agree), "speedup_vs_1gpu": (K / (tp_ms * 1e-3)) / (K / (r["best_ms"] * 1e-3))}
+                    "ranks_agree": bool(ranks_agree), "speedup_vs_1gpu": (K / (tp_ms * 1e-3)) / (K / (r["ms"] * 1e-3))}
           assert ranks_agree, "tensor-parallel ranks produced different tokens"
           mt.close()
       except Exception as e:   # the weak-scaling line must survive a failure of the strong-scaling arm
@@ -529,7 +548,7 @@ def main():
                 "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
                 "dtype": "f32 (fp16 weights, fp32 activations/accumulate/KV)", "data": "synthetic",
                 "config": dict(config, prefill_secs=usage["prompt_secs"], tower_secs=usage["vision_secs"], kernels_per_step=st["kernels_per_decode_step"],
-                               reps=reps, value_wall_check_s=r["wall_value"]),
+                               value_wall_check_s=r["wall_value"]),
                 "clocks": clocks, "gpu_launches": int(r["launches"]),
                 "e2e": {"value": e2e_val, "unit": UNIT, "h2d_bytes_per_step": 16, "d2h_bytes_per_step": 4,
                         "with_logits_d2h_tokens_per_s": 1.0 / r["e2e_logits_s"], "logits_bytes": 4 * tc["vocab_size"]},

@@ -12,9 +12,9 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
 from aha_b200 import B200Model, synth   # noqa: E402
-
-GOLD = os.path.join(ROOT, "tests", "golden")
+from make_golden_full import load       # noqa: E402
 
 
 def chain(m, g, S, prefill_logits):
@@ -32,14 +32,14 @@ def chain(m, g, S, prefill_logits):
 
 def main():
     out = {}
-    g = np.load(os.path.join(GOLD, "full_q06.npz"))
+    g = load("full_q06")
     cfg = synth.get_config("qwen3", "q0.6")
     m = B200Model("qwen3", cfg, synth.make_weights("qwen3", cfg, 0), eos_ids=[], max_ctx=2048, max_prefill=2048)
     ids = synth.synth_text_ids(synth.FULL_Q06_PROMPT, 151000, 21)
     out["q0.6 (1920-token prompt)"] = chain(m, g, len(ids), m.forward_initial(ids, 0)[0, 0])
     m.close()
 
-    g = np.load(os.path.join(GOLD, "full_vl2.npz"))
+    g = load("full_vl2")
     cfg = synth.get_config("qwen3vl", "vl2")
     m = B200Model("qwen3vl", cfg, synth.make_weights("qwen3vl", cfg, 0), eos_ids=[], max_ctx=4096, max_prefill=4096, max_patches=8192)
     pv, grid = m.image_patchify(synth.synth_image(*synth.FULL_VL2_IMAGE, seed=1))
@@ -47,7 +47,7 @@ def main():
     out["vl2 (1080p image + 512 ids)"] = chain(m, g, len(ids), m.forward_initial(ids, 0, [pv, grid, None, None, None])[0, 0])
     m.close()
 
-    g = np.load(os.path.join(GOLD, "full_asr06.npz"))
+    g = load("full_asr06")
     cfg = synth.get_config("qwen3_asr", "asr0.6")
     m = B200Model("qwen3_asr", cfg, synth.make_weights("qwen3_asr", cfg, 0), eos_ids=[], max_ctx=1024, max_frames=3000)
     mel = m.mel_spectrogram(synth.synth_audio(synth.FULL_ASR_SECONDS))

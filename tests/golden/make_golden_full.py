@@ -1,6 +1,6 @@
 """Full-size golden fixtures: ONE oracle forward at each BASELINE.json shape (configs 2, 3, 4), run on the CPU of the
 build container (`python tests/golden/make_golden_full.py [vl2|q0.6|asr0.6 ...]`, minutes each), outputs committed as
-`tests/golden/full_*.npz`.  Weights and inputs are re-derived from the seeds by aha_b200.synth, so the fixtures hold
+`tests/golden/full_<name>.<i>.npz` (one fixture is split over several files so that none reaches 1 MB; `load` joins them).  Weights and inputs are re-derived from the seeds by aha_b200.synth, so the fixtures hold
 only what the GPU tests compare (tests/test_fullsize_gpu.py):
 
   * `prefill_logits` (V) of the last prompt token, full f32;
@@ -11,6 +11,7 @@ only what the GPU tests compare (tests/test_fullsize_gpu.py):
   * Qwen3-ASR: the same for the audio-tower output, and the oracle log-mel checksum.
 
 The oracle is the checker, never the product (oracle/__init__.py)."""
+import glob
 import os
 import sys
 import time
@@ -25,9 +26,36 @@ OUT = os.path.dirname(os.path.abspath(__file__))
 N_STEPS = 8
 SUB = 8
 TOPK = 16
+SHARD_BYTES = 900_000   # float32 logits hardly compress: a fixture file holds at most this many bytes of arrays
 
 # the three workloads; tests/test_fullsize_gpu.py and bench.py build the same inputs from these
 VL2_IMAGE, VL2_TEXT, Q06_PROMPT, ASR_SECONDS = synth.FULL_VL2_IMAGE, synth.FULL_VL2_TEXT, synth.FULL_Q06_PROMPT, synth.FULL_ASR_SECONDS
+
+
+def save(name, out):
+    """The arrays of `out`, in order, as name.0.npz, name.1.npz, ...: a new file whenever the next array would take the current one past
+    SHARD_BYTES."""
+    for f in glob.glob(os.path.join(OUT, f"{name}.*.npz")):
+        os.remove(f)
+    shard, size, i = {}, 0, 0
+    for k, v in out.items():
+        v = np.asarray(v)
+        if shard and size + v.nbytes > SHARD_BYTES:
+            np.savez_compressed(os.path.join(OUT, f"{name}.{i}.npz"), **shard)
+            shard, size, i = {}, 0, i + 1
+        shard[k] = v
+        size += v.nbytes
+    np.savez_compressed(os.path.join(OUT, f"{name}.{i}.npz"), **shard)
+
+
+def load(name):
+    """Every array of fixture `name` (all its files) in one dict."""
+    paths = glob.glob(os.path.join(OUT, f"{name}.*.npz"))
+    assert paths, f"tests/golden/{name}.*.npz is missing: run python tests/golden/make_golden_full.py"
+    g = {}
+    for p in paths:
+        g.update(np.load(p))
+    return g
 
 
 def top2gap(l):
@@ -98,7 +126,7 @@ def vl2():
     out["prefill_logits"] = logits.astype(np.float32)
     out["rope_delta"] = np.int64(m.rope_deltas)
     decode_block(m, logits, len(ids), out)
-    np.savez_compressed(os.path.join(OUT, "full_vl2.npz"), **out)
+    save("full_vl2", out)
 
 
 def q06():
@@ -114,7 +142,7 @@ def q06():
     print(f"  prefill {out['prefill_secs_cpu']:.1f} s", flush=True)
     out["prefill_logits"] = logits.astype(np.float32)
     decode_block(m, logits, len(ids), out)
-    np.savez_compressed(os.path.join(OUT, "full_q06.npz"), **out)
+    save("full_q06", out)
 
 
 def asr06():
@@ -141,7 +169,7 @@ def asr06():
     out["prefill_secs_cpu"] = np.float64(time.perf_counter() - t0)
     out["prefill_logits"] = logits.astype(np.float32)
     decode_block(m, logits, len(ids), out)
-    np.savez_compressed(os.path.join(OUT, "full_asr06.npz"), **out)
+    save("full_asr06", out)
 
 
 if __name__ == "__main__":

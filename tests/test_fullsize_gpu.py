@@ -115,15 +115,12 @@ def test_asr06_config4_30s_audio():
 # the build container by tests/golden/make_golden_full.py and committed as tests/golden/full_*.npz (weights and inputs are
 # re-derived from the same seeds here).  Tolerance: north_star's 1e-3 on every logit; greedy ids must equal the oracle's
 # wherever the oracle's top-1/top-2 gap exceeds 10x the measured error.
-import os
+import sys
 
 from conftest import GOLDEN
 
-
-def _golden(name):
-    p = os.path.join(GOLDEN, name)
-    assert os.path.exists(p), f"{p} is missing: run python tests/golden/make_golden_full.py in the build container"
-    return np.load(p)
+sys.path.insert(0, GOLDEN)
+from make_golden_full import load as _golden  # noqa: E402
 
 
 def _check_chain(m, g, S, prefill_logits, label):
@@ -155,7 +152,7 @@ def _check_chain(m, g, S, prefill_logits, label):
 def test_vl2_1080p_matches_the_full_size_oracle_golden(vl2, impl):
     cfg, m0, m1 = vl2
     m = m1 if impl == 1 else m0
-    g = _golden("full_vl2.npz")
+    g = _golden("full_vl2")
     VL2_IMAGE, VL2_TEXT = synth.FULL_VL2_IMAGE, synth.FULL_VL2_TEXT
     m.clear_cache()
     pv, grid = m.image_patchify(synth.synth_image(*VL2_IMAGE, seed=1))
@@ -176,7 +173,7 @@ def test_vl2_1080p_matches_the_full_size_oracle_golden(vl2, impl):
 @pytest.mark.parametrize("impl", [0, 1, 2])
 def test_q06_2k_matches_the_full_size_oracle_golden(impl):
     Q06_PROMPT = synth.FULL_Q06_PROMPT
-    g = _golden("full_q06.npz")
+    g = _golden("full_q06")
     cfg = synth.get_config("qwen3", "q0.6")
     w = synth.make_weights("qwen3", cfg, 0)
     m = B200Model("qwen3", cfg, w, eos_ids=[], max_ctx=2048, max_prefill=2048, decode_impl=impl)
@@ -192,7 +189,7 @@ def test_q06_2k_matches_the_full_size_oracle_golden(impl):
 
 def test_asr06_30s_matches_the_full_size_oracle_golden():
     ASR_SECONDS = synth.FULL_ASR_SECONDS
-    g = _golden("full_asr06.npz")
+    g = _golden("full_asr06")
     cfg = synth.get_config("qwen3_asr", "asr0.6")
     w = synth.make_weights("qwen3_asr", cfg, 0)
     m = B200Model("qwen3_asr", cfg, w, eos_ids=[], max_ctx=1024, max_frames=3000)
