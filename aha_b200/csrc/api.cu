@@ -281,6 +281,10 @@ std::vector<uint32_t> mm_token_ids(const aha_model* m) {
 void require_no_session(aha_model* m) {
     AHA_REQUIRE(!m->session.open, "a batch session is open on this handle: call aha_b200_batch_close first");
 }
+bool is_stop_token(const aha_model* m, uint32_t t) {
+    for (uint32_t e : m->stop_ids) if (e == t) return true;
+    return false;
+}
 bool env_flag(const char* name, bool dflt) { const char* v = std::getenv(name); return v ? std::atoi(v) != 0 : dflt; }
 int env_int(const char* name, int dflt) { const char* v = std::getenv(name); return v ? std::atoi(v) : dflt; }
 // projections of the batched step: 0 = batched GEMV with the weights in registers, 1 = exact SIMT GEMM (validation twin), 2 = batched GEMV with the
@@ -571,20 +575,6 @@ size_t aha_b200_prefix_match(const uint32_t* cached, size_t n_cached, const uint
 
 uint64_t aha_b200_mm_fingerprint(const aha_mm* mm) { return mm_fingerprint(mm); }
 
-int aha_b200_clear_cache(aha_model* m) {
-    return guarded(m, [&] {
-        AHA_CUDA_CHECK(cudaStreamSynchronize(m->ctx.stream));
-        if (m->session.open) {   // clear_cache ends a batch session too: every sequence's K/V is gone
-            for (auto& sl : m->batch.slots) sl.mapped = 0;
-            m->batch.table_for.clear();
-            m->batch.clear_graphs();
-            m->session = aha_model::BatchSession{};
-            m->text.clear_sampler();
-        }
-        drop_cache(m);
-    });
-}
-
 size_t aha_b200_stop_token_ids(aha_model* m, uint32_t* out, size_t cap) {
     if (!m) return 0;
     for (size_t i = 0; i < m->stop_ids.size() && i < cap && out; ++i) out[i] = m->stop_ids[i];
@@ -648,7 +638,6 @@ void generate_impl(aha_model* m, const uint32_t* ids, size_t seq_len, const aha_
     }
     T.set_sampler(mode, params.temperature, params.top_p, params.top_k, params.repeat_penalty, params.repeat_last_n, params.seed);
     T.set_state(0, 0, 0, 0, draws0);    // empty history: the first token sees no repeat-penalty context
-    auto is_eos = [&](uint32_t t) { for (uint32_t e : m->stop_ids) if (e == t) return true; return false; };
     uint32_t tok = 0;
     if (hit > 0) forward_any(m, ids + hit, seq_len - hit, hit, nullptr, false, nullptr, &tok, true);   // only the tokens the cache does not hold yet
     else forward_any(m, ids, seq_len, 0, mm, true, nullptr, &tok);   // forward_initial + sample_and_push
@@ -657,7 +646,7 @@ void generate_impl(aha_model* m, const uint32_t* ids, size_t seq_len, const aha_
     const double vision_secs = m->last_vision_secs;
     size_t done = 1;
     produced.push_back(tok);
-    bool stop = sink.push(tok, 0) || (eos_on_first && is_eos(tok));   // generate_generic never EOS-checks the first token; the ASR loop does
+    bool stop = sink.push(tok, 0) || (eos_on_first && is_stop_token(m, tok));   // generate_generic never EOS-checks the first token; the ASR loop does
     if (sample_len > 1 && !stop) {
         T.ensure_tokens((int)(seq_len + sample_len));
         DecodeState cur;
@@ -683,7 +672,7 @@ void generate_impl(aha_model* m, const uint32_t* ids, size_t seq_len, const aha_
                 const uint32_t t = m->h_pin[i];
                 ++done;
                 produced.push_back(t);
-                stop = sink.push(t, done - 1) || is_eos(t);   // an EOS token is pushed before the break (generate.rs:139-141)
+                stop = sink.push(t, done - 1) || is_stop_token(m, t);   // an EOS token is pushed before the break (generate.rs:139-141)
             }
             AHA_CUDA_CHECK(cudaStreamSynchronize(m->ctx.stream));
             T.check_ll_abort();
@@ -712,27 +701,6 @@ void generate_impl(aha_model* m, const uint32_t* ids, size_t seq_len, const aha_
 }  // namespace
 
 namespace {
-// One request into slot `slot` of the batch decoder: the reference's forward_initial + sample_and_push on the slot's own page table (swapped into
-// the TextModel for the duration, so tower / M-RoPE / deepstack / sampler-on-prefill are the single-request code), then its decode state, history
-// and sampler move into the slot.  *swapped tells the caller's guard which table is swapped in if this throws.
-uint32_t batch_prefill_slot(aha_model* m, int slot, const aha_batch_request& r, size_t sample_len, int* swapped) {
-    TextModel& T = m->text;
-    BatchDecoder& B = m->batch;
-    B.swap_table(slot); *swapped = slot;
-    m->have_rope_delta = false; m->rope_delta = 0;
-    T.set_sampler(sampling_mode(r.params), r.params.temperature, r.params.top_p, r.params.top_k, r.params.repeat_penalty, r.params.repeat_last_n, r.params.seed);
-    T.set_state(0, 0, 0, 0, 0);
-    uint32_t tok = 0;
-    forward_any(m, r.ids, r.seq_len, 0, r.mm, true, nullptr, &tok, false, true);
-    T.check_sample_error();
-    T.ensure_tokens((int)(r.seq_len + sample_len));       // every page the request can touch is mapped now (the step kernels only read the table)
-    DecodeState cur;
-    AHA_CUDA_CHECK(cudaMemcpy(&cur, T.d_state, sizeof(cur), cudaMemcpyDeviceToHost));
-    B.adopt(slot, tok, (int)r.seq_len, m->kind == aha_model::QWEN3VL ? m->rope_delta : 0, cur.n_draws);
-    B.swap_table(slot); *swapped = -1;
-    return tok;
-}
-
 // ---- continuous batching: the same slots and the same step, with requests joining and leaving between steps -------------------------
 // (new design; the reference's server holds ONE request behind a write lock, server/api.rs:117.)  A finished request's pages go back to the
 // free list at once, so a waiting request can take its place while the others keep decoding.
@@ -746,7 +714,7 @@ void session_release(aha_model* m, int slot) {
     m->batch.clear_graphs();       // the graphs of compositions holding this slot carry its sampler arguments by value
 }
 void session_close(aha_model* m) {
-    if (m->batch.cap) { for (auto& sl : m->batch.slots) sl.mapped = 0; m->batch.table_for.clear(); m->batch.clear_graphs(); }
+    m->batch.reset();
     m->session = aha_model::BatchSession{};
     drop_cache(m);
     m->text.clear_sampler();
@@ -758,14 +726,16 @@ void session_open(aha_model* m) {
     AHA_REQUIRE(T.max_prefill >= kGemvBatchMax, "batch sessions need max_prefill >= 8");
     drop_cache(m);
     m->batch.init(T, kGemvBatchMax);
-    for (auto& sl : m->batch.slots) sl.mapped = 0;
-    m->batch.table_for.clear();
-    m->batch.clear_graphs();
+    m->batch.reset();
     m->session = aha_model::BatchSession{};
     m->session.open = true;
 }
+// One request into a free slot: the reference's forward_initial + sample_and_push on the slot's own page table (swapped into the TextModel
+// for the duration, so tower / M-RoPE / deepstack / sampler-on-prefill are the single-request code), then its decode state, history and
+// sampler move into the slot.
 void session_add(aha_model* m, const aha_batch_request& r, int* slot_out, uint32_t* first_token, int* finished, aha_usage* usage) {
     TextModel& T = m->text;
+    BatchDecoder& B = m->batch;
     AHA_REQUIRE(m->session.open, "no batch session is open (aha_b200_batch_open)");
     AHA_REQUIRE(r.ids && r.seq_len >= 1, "batch_add: the request needs input_ids");
     AHA_REQUIRE((r.params.flags & (AHA_GEN_CONTINUE_RNG | AHA_GEN_REUSE_PREFIX)) == 0, "batch_add: CONTINUE_RNG / REUSE_PREFIX are per-handle states of the single-request calls");
@@ -778,21 +748,30 @@ void session_add(aha_model* m, const aha_batch_request& r, int* slot_out, uint32
                                                   std::to_string(T.free_pages.size() * kPage) + " are free (max_ctx " + std::to_string(T.max_ctx) + ")");
     using clk = std::chrono::steady_clock;
     const auto t0 = clk::now();
-    int swapped = -1;
-    struct Guard {   // a failed prefill leaves the session as it was: own table back in place, the slot's pages back in the pool
-        aha_model* m; int slot; int* swapped; bool ok = false;
-        ~Guard() { if (ok) return; if (*swapped >= 0) m->batch.swap_table(*swapped); session_release(m, slot); m->have_rope_delta = false; m->rope_delta = 0; m->text.clear_sampler(); }
-    } guard{m, slot, &swapped};
     m->session.used[slot] = true;
-    const uint32_t tok = batch_prefill_slot(m, slot, r, sample_len, &swapped);
+    B.swap_table(slot);
+    struct Guard {   // a failed prefill leaves the session as it was: own table back in place, the slot's pages back in the pool
+        aha_model* m; int slot; bool ok = false;
+        ~Guard() { if (ok) return; m->batch.swap_table(slot); session_release(m, slot); m->have_rope_delta = false; m->rope_delta = 0; m->text.clear_sampler(); }
+    } guard{m, slot};
+    m->have_rope_delta = false; m->rope_delta = 0;
+    T.set_sampler(sampling_mode(r.params), r.params.temperature, r.params.top_p, r.params.top_k, r.params.repeat_penalty, r.params.repeat_last_n, r.params.seed);
+    T.set_state(0, 0, 0, 0, 0);
+    uint32_t tok = 0;
+    forward_any(m, r.ids, r.seq_len, 0, r.mm, true, nullptr, &tok, false, true);
+    T.check_sample_error();
+    T.ensure_tokens((int)(r.seq_len + sample_len));       // every page the request can touch is mapped now (the step kernels only read the table)
+    DecodeState cur;
+    AHA_CUDA_CHECK(cudaMemcpy(&cur, T.d_state, sizeof(cur), cudaMemcpyDeviceToHost));
+    B.adopt(slot, tok, (int)r.seq_len, m->kind == aha_model::QWEN3VL ? m->rope_delta : 0, cur.n_draws);
+    B.swap_table(slot);
     guard.ok = true;
-    m->text.clear_sampler();
-    m->batch.table_for.clear();
-    m->batch.clear_graphs();
+    T.clear_sampler();
+    B.table_for.clear();
+    B.clear_graphs();
     m->session.budget[slot] = sample_len;
     m->session.produced[slot] = 1;
-    bool stop = sample_len == 1;
-    if ((r.params.flags & AHA_GEN_EOS_ON_FIRST) != 0) for (uint32_t e : m->stop_ids) if (e == tok) stop = true;
+    const bool stop = sample_len == 1 || ((r.params.flags & AHA_GEN_EOS_ON_FIRST) != 0 && is_stop_token(m, tok));
     if (usage) {
         *usage = aha_usage{};
         usage->prompt_tokens = (uint32_t)r.seq_len; usage->completion_tokens = 1;
@@ -807,6 +786,7 @@ size_t session_step(aha_model* m, uint32_t* tokens_out, int32_t* status_out) {
     std::vector<int> act;
     for (int i = 0; i < kGemvBatchMax; ++i) { status_out[i] = 0; tokens_out[i] = 0; if (m->session.used[i]) act.push_back(i); }
     if (act.empty()) return 0;
+    // AHA_BATCH_GRAPH=0: eager launches (A/B twin of the per-composition graphs)
     m->batch.step(act, env_int("AHA_BATCH_GEMV", kBatchGemvDefault), env_flag("AHA_BATCH_GRAPH", true));
     uint32_t h_tok[kGemvBatchMax];
     AHA_CUDA_CHECK(cudaMemcpyAsync(h_tok, m->batch.d_tok, sizeof(h_tok), cudaMemcpyDeviceToHost, m->ctx.stream));
@@ -816,98 +796,71 @@ size_t session_step(aha_model* m, uint32_t* tokens_out, int32_t* status_out) {
         const uint32_t t = h_tok[slot];
         tokens_out[slot] = t;
         m->session.produced[slot] += 1;
-        bool stop = m->session.produced[slot] >= m->session.budget[slot];
-        for (uint32_t e : m->stop_ids) if (e == t) stop = true;     // an EOS token is delivered, then the request ends (generate.rs:139-141)
+        // an EOS token is delivered, then the request ends (generate.rs:139-141)
+        const bool stop = m->session.produced[slot] >= m->session.budget[slot] || is_stop_token(m, t);
         status_out[slot] = stop ? 2 : 1;
     }
     for (int slot : act) if (status_out[slot] == 2) session_release(m, slot);
-    // sampler errors surface after the bookkeeping so that the slots stay consistent
-    {
-        TextModel& T = m->text;
-        if (T.d_sample_err) {
-            int e = 0;
-            AHA_CUDA_CHECK(cudaMemcpy(&e, T.d_sample_err, sizeof(int), cudaMemcpyDeviceToHost));
-            if (e) { cudaMemset(T.d_sample_err, 0, sizeof(int)); throw std::runtime_error("sampler: the token weights are all zero or not finite (rand::distr::weighted::WeightedIndex::new fails in the reference)"); }
-        }
-    }
+    m->text.check_sample_flag();   // sampler errors surface after the bookkeeping so that the slots stay consistent
     return act.size();
 }
 
-// Static batching: n independent requests, each prefilled on its own page table, then decoded in lockstep (batch_decode.cuh).  Every
-// request follows generate_generic's rules on its own (first token never EOS-checked, an EOS token is pushed and ends THAT request, its
-// own sampler / seed / repeat-penalty history) and so yields exactly the tokens aha_b200_generate would yield for it alone.
+// Static batching: a batch session whose n requests are all added before the first step, then stepped until every one has finished.
+// Every request follows generate_generic's rules on its own (first token never EOS-checked, an EOS token is pushed and ends THAT request,
+// its own sampler / seed / repeat-penalty history) and so yields exactly the tokens aha_b200_generate would yield for it alone.
 void generate_batch_impl(aha_model* m, const aha_batch_request* reqs, size_t n, uint32_t* out_tokens, size_t cap, size_t* n_out, aha_usage* usage) {
     TextModel& T = m->text;
     require_no_session(m);
     AHA_REQUIRE(n >= 1 && n <= (size_t)kGemvBatchMax, "generate_batch: 1 to 8 requests");
     AHA_REQUIRE(T.tp_world == 1, "generate_batch is single-GPU (run one batch per tensor-parallel group member instead)");
     AHA_REQUIRE(T.max_prefill >= kGemvBatchMax, "generate_batch needs max_prefill >= 8");
-    using clk = std::chrono::steady_clock;
-    std::vector<size_t> sample_len(n);
     size_t pages = 0;
     for (size_t i = 0; i < n; ++i) {
         AHA_REQUIRE(reqs[i].ids && reqs[i].seq_len >= 1, "generate_batch: every request needs input_ids");
-        sample_len[i] = std::max<size_t>(reqs[i].params.max_tokens, 1);
-        AHA_REQUIRE(cap >= sample_len[i], "out_tokens capacity (per request) is smaller than max_tokens");
+        const size_t sample_len = std::max<size_t>(reqs[i].params.max_tokens, 1);
+        AHA_REQUIRE(cap >= sample_len, "out_tokens capacity (per request) is smaller than max_tokens");
         AHA_REQUIRE((reqs[i].params.flags & (AHA_GEN_CONTINUE_RNG | AHA_GEN_REUSE_PREFIX)) == 0, "generate_batch: CONTINUE_RNG / REUSE_PREFIX are per-handle states of the single-request calls");
-        pages += (reqs[i].seq_len + sample_len[i] + kPage - 1) / kPage;
+        pages += (reqs[i].seq_len + sample_len + kPage - 1) / kPage;
         n_out[i] = 0;
         if (usage) usage[i] = aha_usage{};
     }
+    // the whole batch is refused before any prefill runs, rather than by the session_add that would not fit
     AHA_REQUIRE(pages <= (size_t)T.num_pages, "the requests of the batch need " + std::to_string(pages * kPage) + " tokens of KV capacity, max_ctx is " + std::to_string(T.max_ctx));
-    const int simt = env_int("AHA_BATCH_GEMV", kBatchGemvDefault);
-    const bool use_graph = env_flag("AHA_BATCH_GRAPH", true);   // 0 = eager launches (A/B twin of the per-composition graphs)
-    BatchDecoder& B = m->batch;
-    drop_cache(m);
-    B.init(T, kGemvBatchMax);
-    for (auto& sl : B.slots) sl.mapped = 0;
-    B.table_for.clear();
-    B.clear_graphs();
-    int swapped = -1;
-    struct Reset {   // whatever happens, the handle is left as after clear_cache(), with its own page table in place
-        aha_model* m; BatchDecoder* B; int* swapped;
-        ~Reset() { if (*swapped >= 0) B->swap_table(*swapped); drop_cache(m); m->text.clear_sampler(); for (auto& sl : B->slots) sl.mapped = 0; B->clear_graphs(); }
-    } reset{m, &B, &swapped};
-    auto is_eos = [&](uint32_t t) { for (uint32_t e : m->stop_ids) if (e == t) return true; return false; };
-
-    // ---- prefill, one request after the other (each is the reference's forward_initial + sample_and_push)
-    std::vector<int> act;
-    std::vector<clk::time_point> t_first(n);
+    session_open(m);
+    struct Close {   // whatever happens, the handle is left as after clear_cache(), with its own page table in place
+        aha_model* m;
+        ~Close() { session_close(m); }
+    } close{m};
+    int req_of[kGemvBatchMax];   // request held by each slot: a request finished by its prefill hands its slot to the next one
     for (size_t i = 0; i < n; ++i) {
-        const aha_batch_request& r = reqs[i];
-        const auto t0 = clk::now();
-        const uint32_t tok = batch_prefill_slot(m, (int)i, r, sample_len[i], &swapped);
-        t_first[i] = clk::now();
-        out_tokens[i * cap] = tok; n_out[i] = 1;
-        if (usage) {
-            usage[i].prompt_tokens = (uint32_t)r.seq_len;
-            usage[i].prompt_secs = std::chrono::duration<double>(t_first[i] - t0).count();
-            usage[i].vision_secs = m->last_vision_secs;
-        }
-        const bool stop = (r.params.flags & AHA_GEN_EOS_ON_FIRST) != 0 && is_eos(tok);
-        if (sample_len[i] > 1 && !stop) act.push_back((int)i);
+        int slot = -1, fin = 0;
+        session_add(m, reqs[i], &slot, out_tokens + i * cap, &fin, usage ? usage + i : nullptr);
+        req_of[slot] = (int)i;
+        n_out[i] = 1;
     }
-    // ---- decode in lockstep; a request leaves the batch at its EOS token or at max_tokens
+    using clk = std::chrono::steady_clock;
     const auto t_dec = clk::now();
-    std::vector<uint32_t> h_tok(kGemvBatchMax);
-    while (!act.empty()) {
-        B.step(act, simt, use_graph);
-        AHA_CUDA_CHECK(cudaMemcpyAsync(h_tok.data(), B.d_tok, kGemvBatchMax * sizeof(uint32_t), cudaMemcpyDeviceToHost, m->ctx.stream));
-        AHA_CUDA_CHECK(cudaStreamSynchronize(m->ctx.stream));
-        T.check_sample_error();
-        std::vector<int> next;
-        for (int slot : act) {
-            const uint32_t t = h_tok[slot];
-            out_tokens[(size_t)slot * cap + n_out[slot]] = t;
-            n_out[slot] += 1;
-            if (!(is_eos(t) || n_out[slot] >= sample_len[slot])) next.push_back(slot);
-            else if (usage) usage[slot].completion_secs = std::chrono::duration<double>(clk::now() - t_dec).count();
+    uint32_t tok[kGemvBatchMax];
+    int32_t status[kGemvBatchMax];
+    while (session_step(m, tok, status) > 0) {
+        for (int slot = 0; slot < kGemvBatchMax; ++slot) {
+            if (status[slot] == 0) continue;
+            const size_t i = (size_t)req_of[slot];
+            out_tokens[i * cap + n_out[i]++] = tok[slot];
+            if (status[slot] == 2 && usage) usage[i].completion_secs = std::chrono::duration<double>(clk::now() - t_dec).count();
         }
-        act.swap(next);
     }
     if (usage) for (size_t i = 0; i < n; ++i) usage[i].completion_tokens = (uint32_t)n_out[i];
 }
 }  // namespace
+
+int aha_b200_clear_cache(aha_model* m) {
+    return guarded(m, [&] {
+        AHA_CUDA_CHECK(cudaStreamSynchronize(m->ctx.stream));
+        if (m->session.open) session_close(m);   // clear_cache ends a batch session too: every sequence's K/V is gone
+        else drop_cache(m);
+    });
+}
 
 int aha_b200_batch_open(aha_model* m) { return guarded(m, [&] { session_open(m); }); }
 

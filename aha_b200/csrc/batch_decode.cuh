@@ -40,13 +40,19 @@ struct BatchDecoder {
     DecodeAttnArgs* d_attn = nullptr;    // [L][cap] attention arguments of the current active list
     std::vector<BatchSlot> slots;
     std::vector<int> table_for;          // active list the attention table was built for
-    // One CUDA graph per composition of the batch (the active list changes only when a request finishes): ~170 launches per step become one.
-    // The graphs hold the requests' sampler parameters by value, so they live for one generate_batch call.
+    // One CUDA graph per composition of the batch (the active list changes only when a request joins or leaves): ~170 launches per step become one.
+    // The graphs hold the requests' sampler parameters by value, so they are dropped whenever a request leaves its slot.
     struct StepGraph { std::vector<int> act; int simt; cudaGraphExec_t exec; uint64_t kernels; };
     std::vector<StepGraph> graphs;
     void clear_graphs() {
         for (auto& g : graphs) if (g.exec) cudaGraphExecDestroy(g.exec);
         graphs.clear();
+    }
+    // no sequence in any slot (their pages go back with the model's reset_pages), no attention table, no graphs
+    void reset() {
+        for (auto& s : slots) { s.mapped = 0; s.samp_active = false; }
+        table_for.clear();
+        clear_graphs();
     }
 
     void init(TextModel& t, int n) {

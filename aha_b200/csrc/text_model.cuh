@@ -926,7 +926,11 @@ struct TextModel {
         ctx->cnt.kernels++;
     }
     void check_sample_error() {
-        if (!d_sample_err || !samp_active) return;
+        if (samp_active) check_sample_flag();
+    }
+    // the error flag whichever sampler set it: a batch step samples with each slot's own sampler, not the model's active one
+    void check_sample_flag() {
+        if (!d_sample_err) return;
         int e = 0;
         AHA_CUDA_CHECK(cudaMemcpy(&e, d_sample_err, sizeof(int), cudaMemcpyDeviceToHost));
         if (e) {

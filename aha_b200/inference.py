@@ -209,6 +209,14 @@ class B200Model:
                                                 C.byref(n), C.byref(u)))
         return [int(out[i]) for i in range(n.value)], self._usage(u)
 
+    def _batch_request(self, input_ids, data, params):
+        """-> (L.BatchRequest, keep): `keep` holds the buffers the request points into; it must outlive the call that reads it."""
+        ids = self._ids(input_ids)
+        mm, k = self._mm(data)
+        req = L.BatchRequest(ids=ids.ctypes.data_as(C.POINTER(C.c_uint32)), seq_len=ids.size,
+                             mm=C.pointer(mm) if mm is not None else None, params=params)
+        return req, (ids, mm, k)
+
     def generate_batch(self, requests):
         """Static batching (aha_b200_generate_batch): requests = [dict(input_ids=..., data=None, max_tokens=..., temperature=..., top_p=...,
         top_k=..., repeat_penalty=..., repeat_last_n=..., seed=...), ...] (at most 8) decoded in lockstep on this handle.
@@ -218,14 +226,10 @@ class B200Model:
         keep = []
         cap = 1
         for i, r in enumerate(requests):
-            ids = self._ids(r["input_ids"])
-            mm, k = self._mm(r.get("data"))
-            keep += [ids, mm, k]
-            arr[i].ids = ids.ctypes.data_as(C.POINTER(C.c_uint32))
-            arr[i].seq_len = ids.size
-            arr[i].mm = C.pointer(mm) if mm is not None else None
-            arr[i].params = self._gen_params(r.get("max_tokens", 1024), r.get("temperature", 0.0), r.get("top_p"), r.get("top_k"),
-                                             r.get("repeat_penalty", 1.0), r.get("repeat_last_n", 64), r.get("seed", 299792458), r.get("flags", 0))
+            p = self._gen_params(r.get("max_tokens", 1024), r.get("temperature", 0.0), r.get("top_p"), r.get("top_k"),
+                                 r.get("repeat_penalty", 1.0), r.get("repeat_last_n", 64), r.get("seed", 299792458), r.get("flags", 0))
+            arr[i], k = self._batch_request(r["input_ids"], r.get("data"), p)
+            keep.append(k)
             cap = max(cap, r.get("max_tokens", 1024))
         out = (C.c_uint32 * (n * cap))()
         n_out = (C.c_size_t * n)()
@@ -240,13 +244,8 @@ class B200Model:
     def batch_add(self, input_ids, data=None, max_tokens=1024, temperature=0.0, top_p=None, top_k=None, repeat_penalty=1.0, repeat_last_n=64,
                   seed=299792458, flags=0):
         """Prefill one request into a free slot -> (slot, first token, finished)."""
-        ids = self._ids(input_ids)
-        mm, _keep = self._mm(data)
-        req = L.BatchRequest()
-        req.ids = ids.ctypes.data_as(C.POINTER(C.c_uint32))
-        req.seq_len = ids.size
-        req.mm = C.pointer(mm) if mm is not None else None
-        req.params = self._gen_params(max_tokens, temperature, top_p, top_k, repeat_penalty, repeat_last_n, seed, flags)
+        req, _keep = self._batch_request(input_ids, data,
+                                         self._gen_params(max_tokens, temperature, top_p, top_k, repeat_penalty, repeat_last_n, seed, flags))
         slot, fin, tok = C.c_int32(-1), C.c_int32(0), C.c_uint32(0)
         u = L.Usage()
         self._check(self._lib.aha_b200_batch_add(self._h, C.byref(req), C.byref(slot), C.byref(tok), C.byref(fin), C.byref(u)))
